@@ -318,11 +318,12 @@ def measure_device_loop(model, args, dev, rank, world, K, W, flush, n_pool=8, sa
     barrier()
     wall0 = time.perf_counter()
     loop0.record()
+    last = None
     for i in range(K):
         if flush is not None:
             flush.zero_()
         ev[i][0].record()
-        device_step(W + i)
+        last = device_step(W + i)
         ev[i][1].record()
         if sync_each_step:
             torch.cuda.synchronize()
@@ -331,7 +332,22 @@ def measure_device_loop(model, args, dev, rank, world, K, W, flush, n_pool=8, sa
     wall = time.perf_counter() - wall0
     step_ms = [a.elapsed_time(b) for a, b in ev]
     return {"step_ms": step_ms, "sum_ms": sum(step_ms), "loop_ms": loop0.elapsed_time(loop1), "wall_s": wall,
-            "host_batches": host_batches, "device_step": device_step, "barrier": barrier}
+            "host_batches": host_batches, "device_step": device_step, "barrier": barrier, "last": last}
+
+
+def dump_outputs(model, last, out_dir, rank):
+    """Write what the last timed step handed back (loss, accuracy, logged learning rate, multi-step loss weights and
+    the per-task target logits, i.e. what ``run_train_iter`` returns) as ``<out_dir>/<name>.npy`` so that two builds
+    can be compared output for output.  Must run before anything else reuses the engine's result buffers."""
+    import numpy as np
+    losses, preds = model._finish(*last)
+    losses["learning_rate"] = model._logged_lr(0)
+    arrays = {k: np.asarray(v, dtype=np.float64 if isinstance(v, float) else np.float32) for k, v in losses.items()}
+    arrays["logits"] = np.stack(preds).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if rank == 0 else "_rank%d" % rank
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
 
 
 def gather_rank_stats(step_ms, loop_ms, coll_us, dev, world):
@@ -426,6 +442,8 @@ def main():
                     help="weak: every GPU holds the config's meta-batch; strong: the config's meta-batch is split over the GPUs")
     ap.add_argument("--no-flush", action="store_true", help="diagnostic: do not flush L2 between timed steps")
     ap.add_argument("--sync-each-step", action="store_true", help="diagnostic: synchronize after every timed step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (same arguments, same inputs)")
     cli = ap.parse_args()
 
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner to fd 1 when
@@ -478,6 +496,8 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     r = measure_device_loop(model, args, dev, rank, world, K, W, flush, sampler=sampler, sync_each_step=cli.sync_each_step)
     step_ms, device_step, barrier = r["step_ms"], r["device_step"], r["barrier"]
+    if cli.dump_outputs:
+        dump_outputs(model, r["last"], cli.dump_outputs, rank)
     host_batches = r["host_batches"]
     n_pool = len(host_batches)
     pinned_batches = [tuple(t.pin_memory() for t in hb) for hb in host_batches]

@@ -35,6 +35,10 @@ from howtotrainyourmamlpytorch_b200.utils.parser_utils import args_from_json  # 
 from oracle import maml_oracle as O  # noqa: E402
 
 REF = "/root/reference"
+# intra-op threads of every reference / oracle run in this script: fp32 CPU convolutions split their reductions by
+# thread, so the CPU tests that compare the fp32 oracle with these fixtures run with the same count
+# (tests/test_oracle_golden.py)
+THREADS = 8
 
 _TINY = dict(image_height=20, image_width=20, image_channels=3, cnn_num_filters=16,
              num_classes_per_set=3, num_samples_per_class=2, num_target_samples=2,
@@ -253,6 +257,95 @@ def write_episode_fixture():
     return path
 
 
+class _CallRecorder(object):
+    """Stands in for a model: forwards everything to ``model`` and logs the public calls an experiment driver makes on
+    it (method, keyword arguments as JSON, what came back)."""
+
+    def __init__(self, model, root):
+        self._model, self._root, self.calls = model, root, []
+
+    def __getattr__(self, name):
+        attr = getattr(self._model, name)
+        if name not in ("run_train_iter", "run_validation_iter", "save_model", "load_model"):
+            return attr
+
+        def call(*args, **kwargs):
+            assert not args, "%s called with positional arguments" % name
+            rec = {"method": name, "kwargs": {}}
+            for k, v in kwargs.items():
+                if k == "data_batch":
+                    rec["kwargs"][k] = [{"type": type(t).__name__, "dtype": str(t.dtype), "shape": list(t.shape)} for t in v]
+                elif k == "model_save_dir":
+                    rec["kwargs"][k] = os.path.relpath(v, self._root)
+                elif k == "state":
+                    rec["kwargs"][k] = {sk: sv for sk, sv in v.items() if isinstance(sv, (int, float, str))}
+                else:
+                    rec["kwargs"][k] = v
+            with contextlib.redirect_stdout(io.StringIO()):
+                out = attr(**kwargs)
+            if name in ("run_train_iter", "run_validation_iter"):
+                rec["losses"] = {k: float(v) for k, v in out[0].items()}
+            elif name == "load_model":
+                rec["state"] = {sk: sv for sk, sv in out.items() if isinstance(sv, (int, float, str))}
+            self.calls.append(rec)
+            return out
+        return call
+
+
+def write_builder_fixture(case="tiny_maml"):
+    """The calls the reference's own ``ExperimentBuilder`` (experiment_builder.py) makes on a model, recorded while it
+    drives the reference's ``MAMLFewShotClassifier`` on the first recorded batch of ``case``: ``train_iteration`` (numpy
+    episodes), ``evaluation_iteration`` (torch episodes), ``save_models`` after one iteration, and a second builder that
+    resumes from ``latest`` -> tests/golden/experiment_builder_<case>.json.  The GPU test replays them on this repo's
+    class."""
+    import shutil
+    import tempfile
+    import warnings
+    import tqdm
+    warnings.filterwarnings("ignore")
+    sys.path.insert(0, REF)
+    sys.argv = [sys.argv[0]]
+    import experiment_builder as ref_builder  # noqa: the reference, unmodified
+
+    class _Data(object):                       # stands in for MetaLearningSystemDataLoader (no dataset on disk)
+        def __init__(self, args, current_iter):
+            self.dataset = type("D", (), {"seed": {"train": 0, "val": 0}})()
+
+    args, _, iters = make_args(case)
+    g = np.load(os.path.join(ROOT, "tests", "golden", case + ".npz"))
+    xs, xt, ys, yt = (torch.from_numpy(g["it0/" + n]) for n in ("xs", "xt", "ys", "yt"))
+    tmp = tempfile.mkdtemp()
+    try:
+        args.experiment_name = os.path.join(tmp, "exp")
+        args.continue_from_epoch = "from_scratch"
+        args.max_models_to_save = 2
+        args.total_epochs_before_pause = 1
+        model = build_reference(args, torch.float32)
+        model.load_state_dict({k[len("state/"):]: torch.from_numpy(g[k]) for k in g.files if k.startswith("state/")})
+        rec = _CallRecorder(model, tmp)
+        with contextlib.redirect_stdout(io.StringIO()):
+            eb = ref_builder.ExperimentBuilder(args=args, data=_Data, model=rec, device=torch.device("cpu"))
+        with contextlib.redirect_stdout(io.StringIO()), tqdm.tqdm(total=2, disable=True) as pbar:
+            _, _, it = eb.train_iteration(train_sample=(xs.numpy(), xt.numpy(), ys.numpy(), yt.numpy(), 0), sample_idx=0,
+                                          epoch_idx=float(iters[0][0]), total_losses={}, current_iter=0, pbar_train=pbar)
+            eb.evaluation_iteration(val_sample=(xs, xt, ys, yt, 0), total_losses={}, pbar_val=pbar, phase="val")
+            eb.state["current_iter"] = it
+            eb.save_models(model=rec, epoch=0, state=eb.state)
+        saved = sorted(os.listdir(eb.saved_models_filepath))
+        args.continue_from_epoch = "latest"
+        rec2 = _CallRecorder(build_reference(args, torch.float32), tmp)
+        with contextlib.redirect_stdout(io.StringIO()):
+            ref_builder.ExperimentBuilder(args=args, data=_Data, model=rec2, device=torch.device("cpu"))
+        out = {"case": case, "calls": rec.calls, "saved_models": saved, "resume_calls": rec2.calls}
+    finally:
+        shutil.rmtree(tmp)
+    path = os.path.join(ROOT, "tests", "golden", "experiment_builder_%s.json" % case)
+    with open(path, "w") as fh:
+        json.dump(out, fh, indent=1, sort_keys=True)
+        fh.write("\n")
+    return path
+
+
 def check_against_oracle(args, blob, iters, kind=KIND):
     """Immediately validate both restatements against what was just generated."""
     state = {k[len("state/"):]: torch.from_numpy(v) for k, v in blob.items() if k.startswith("state/")}
@@ -289,12 +382,15 @@ def check_against_oracle(args, blob, iters, kind=KIND):
 def main():
     os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
     which = sys.argv[1:] or list(CASES.keys())
-    torch.set_num_threads(8)
+    torch.set_num_threads(THREADS)
     if "--episodes" in which:
         print(write_episode_fixture())
         return
     if "--checkpoint" in which:
         print(write_reference_checkpoint("tiny_pp"))
+        return
+    if "--builder" in which:
+        print(write_builder_fixture("tiny_maml"))
         return
     for case in which:
         args, argdict, iters = make_args(case)

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import ALL_CASES, BERNOULLI_CASES, BIG_CASES, TINY_CASES, load_golden, grad_tolerance
+from conftest import ALL_CASES, BERNOULLI_CASES, BIG_CASES, GOLDEN_DIR, TINY_CASES, load_golden, grad_tolerance
 from engine_layout import geometry, grid_to_nchw, flat_to_nchw, theta_to_ref, rel_err
 from oracle import maml_oracle as O
 
@@ -47,10 +47,14 @@ def _count_exact_ties(fwd_blocks):
 
 @pytest.mark.parametrize("case", ["tiny_pp", "tiny_maml", "tiny_odd", "tiny_bern"])
 def test_stagewise_against_oracle(case, cuda_device):
-    """Every materialised intermediate of task 0 against the autograd-free oracle (fp32).  ``tiny_bern`` runs
-    Bernoulli(0.93) binary images (the distribution bench.py uses): thousands of pooling windows with EXACT ties,
+    """Every materialised intermediate of task 0 against the autograd-free oracle, evaluated in fp64.  ``tiny_bern``
+    runs Bernoulli(0.93) binary images (the distribution bench.py uses): thousands of pooling windows with EXACT ties,
     which F.max_pool2d resolves first-max-wins -- a tie resolved differently routes the gradient to another pixel and
-    shows up as an O(1) error in dz / dp of that block."""
+    shows up as an O(1) error in dz / dp of that block.  The oracle runs in fp64: on ``tiny_bern`` its fp32
+    evaluation is itself farther from exact than these tolerances (up to 4e-5 of max-norm on the inner-loop weights,
+    varying with the host's CPU thread count, and one near-tie resolved the other way, which moves a final gradient by
+    4e-3 of max-norm), while the engine sits within 0.3x of these tolerances of the fp64 values on every case
+    (measured on a B200)."""
     g = load_golden(case)
     a = g.args
     m = _model(g, cuda_device)
@@ -58,7 +62,7 @@ def test_stagewise_against_oracle(case, cuda_device):
     epoch = g.iters[0][0]
     losses, preds, grads = m.meta_gradient(batch, epoch)
     eng = m._engine
-    ref = O.manual_train_iter(g.state(), a, batch, epoch, keep_intermediates=True)
+    ref = O.manual_train_iter(g.state(torch.float64), a, batch, epoch, keep_intermediates=True)
     inter = [x for x in ref["intermediates"] if "theta" in x and x["task"] == 0][0]
     tang = {x["step"]: x for x in ref["intermediates"] if "Hu" in x and x["task"] == 0}
     geo, (ph, pw) = geometry(a)
@@ -715,58 +719,55 @@ def test_device_trace(cuda_device):
     assert max(starts) - min(starts) < 1e9           # nanoseconds: one tiny iteration spans far less than a second
 
 
-def test_reference_experiment_builder_drives_the_class(cuda_device, tmp_path, monkeypatch):
-    """Level B0 as the reference uses it: the UNMODIFIED ``ExperimentBuilder`` (reference experiment_builder.py:102-164,
-    190-206, staged under baseline/_ref) runs ``train_iteration`` / ``evaluation_iteration`` / ``save_models`` on THIS
-    repo's ``MAMLFewShotClassifier`` -- losses dict keys survive ``float()``, checkpoints are written through
-    ``save_model`` and found again by ``load_model``."""
-    import sys
-    import tqdm
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.exists(os.path.join(ref_dir, "experiment_builder.py")):
-        pytest.skip("baseline/_ref is not staged")
+def test_reference_experiment_builder_drives_the_class(cuda_device, tmp_path):
+    """Level B0 as the reference uses it.  ``tests/golden/experiment_builder_tiny_maml.json`` holds every call the
+    UNMODIFIED reference ``ExperimentBuilder`` makes on a model (``train_iteration`` with numpy episodes,
+    ``evaluation_iteration`` with torch episodes, ``save_models``, and a second builder resuming from ``latest``),
+    recorded while it drove the reference's own class (``oracle/gen_golden.py --builder``).  Replayed on THIS repo's
+    ``MAMLFewShotClassifier``: the same keyword arguments are accepted, the losses dicts carry the reference's keys and
+    values (the builder folds every entry into its summaries with ``float()``), the checkpoints land under the same names
+    and ``load_model`` finds them again."""
+    import json
     from howtotrainyourmamlpytorch_b200 import MAMLFewShotClassifier
-    g = load_golden("tiny_maml")
+    with open(os.path.join(GOLDEN_DIR, "experiment_builder_tiny_maml.json")) as fh:
+        rec = json.load(fh)
+    g = load_golden(rec["case"])
     a = g.args
-    monkeypatch.chdir(tmp_path)
-    monkeypatch.setattr(sys, "argv", ["x"])
-    sys.path.insert(0, ref_dir)
-    saved_utils = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "utils" or k.startswith("utils.")}
-    try:
-        import experiment_builder as ref_builder      # the reference, unmodified
+    episodes = g.batch(0)
 
-        class _Data(object):                           # stands in for MetaLearningSystemDataLoader (data.py: out of scope)
-            def __init__(self, args, current_iter):
-                self.dataset = type("D", (), {"seed": {"train": 0, "val": 0}})()
+    def replay(model, call):
+        kw = dict(call["kwargs"])
+        if "data_batch" in kw:
+            assert [list(t.shape) for t in episodes] == [d["shape"] for d in kw["data_batch"]]
+            kw["data_batch"] = tuple(t.numpy() if d["type"] == "ndarray" else t for t, d in zip(episodes, kw["data_batch"]))
+        if "model_save_dir" in kw:
+            kw["model_save_dir"] = os.path.join(str(tmp_path), kw["model_save_dir"])
+        if call["method"] == "save_model":
+            os.makedirs(os.path.dirname(kw["model_save_dir"]), exist_ok=True)
+            kw["state"] = dict(kw["state"])
+        return getattr(model, call["method"])(**kw)
 
-        a.experiment_name = os.path.join(str(tmp_path), "exp")
-        a.continue_from_epoch = "from_scratch"
-        a.max_models_to_save = 2
-        a.total_epochs_before_pause = 1
-        model = MAMLFewShotClassifier(im_shape=(2, a.image_channels, a.image_height, a.image_width), device=cuda_device, args=a)
-        model.load_state_dict(g.state())
-        eb = ref_builder.ExperimentBuilder(args=a, data=_Data, model=model, device=cuda_device)
-        xs, xt, ys, yt = g.batch(0)
-        with tqdm.tqdm(total=2) as pbar:
-            train_losses, total_losses, it = eb.train_iteration(train_sample=(xs.numpy(), xt.numpy(), ys.numpy(), yt.numpy(), 0),
-                                                                sample_idx=0, epoch_idx=0.0, total_losses={}, current_iter=0,
-                                                                pbar_train=pbar)
-            val_losses, val_total = eb.evaluation_iteration(val_sample=(xs, xt, ys, yt, 0), total_losses={}, pbar_val=pbar,
-                                                            phase="val")
-        assert it == 1
-        assert abs(train_losses["train_loss_mean"] - g.scalar("loss", 0)) <= 1e-4 * abs(g.scalar("loss", 0))
-        assert "train_accuracy_mean" in train_losses and "train_learning_rate_mean" in train_losses
-        assert "val_loss_mean" in val_losses and np.isfinite(val_losses["val_loss_mean"])
-        eb.state["current_iter"] = 1
-        eb.save_models(model=model, epoch=0, state=eb.state)
-        assert os.path.exists(os.path.join(eb.saved_models_filepath, "train_model_latest"))
-        m2 = MAMLFewShotClassifier(im_shape=(2, a.image_channels, a.image_height, a.image_width), device=cuda_device, args=a)
-        st = m2.load_model(model_save_dir=eb.saved_models_filepath, model_name="train_model", model_idx="latest")
-        assert st["current_iter"] == 1
-        for k, v in model.state_dict().items():
-            assert torch.equal(v.cpu(), m2.state_dict()[k].cpu()), k
-    finally:
-        sys.path.remove(ref_dir)
-        for k in [k for k in sys.modules if k == "utils" or k.startswith("utils.") or k == "experiment_builder"]:
-            sys.modules.pop(k)
-        sys.modules.update(saved_utils)
+    model = _model(g, cuda_device)
+    for call in rec["calls"]:
+        out = replay(model, call)
+        if "losses" not in call:
+            continue
+        losses, _ = out
+        assert sorted(losses) == sorted(call["losses"]), call["method"]
+        got, want = {k: float(v) for k, v in losses.items()}, call["losses"]
+        train = call["method"] == "run_train_iter"
+        # validation runs after the Adam step: noise-level gradient elements move differently through Adam's first step
+        # (see test_train_iterations_post_state), so its loss agrees to ~1e-4 and one target prediction may flip
+        assert abs(got["loss"] - want["loss"]) <= (1e-4 if train else 1e-3) * abs(want["loss"]), (call["method"], got, want)
+        assert abs(got["accuracy"] - want["accuracy"]) <= (1e-6 if train else 0.06), (call["method"], got, want)
+        for k in want:
+            if k.startswith("loss_importance_vector") or k == "learning_rate":
+                assert abs(got[k] - want[k]) <= 1e-7, (k, got[k], want[k])
+    saved_dir = os.path.join(str(tmp_path), rec["resume_calls"][0]["kwargs"]["model_save_dir"])
+    assert sorted(os.listdir(saved_dir)) == rec["saved_models"]
+    m2 = MAMLFewShotClassifier(im_shape=(2, a.image_channels, a.image_height, a.image_width), device=cuda_device, args=a)
+    for call in rec["resume_calls"]:
+        st = replay(m2, call)
+        assert {k: st[k] for k in call["state"]} == call["state"]
+    for k, v in model.state_dict().items():
+        assert torch.equal(v.cpu(), m2.state_dict()[k].cpu()), k
